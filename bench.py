@@ -4,7 +4,7 @@ iterations, batch 4096 per GPU (weak scaling over 1/2/4/8 B200; one process per 
 int64 error counters per step, as sim_ber's replicas do: /root/reference/src/sionna/phy/utils/misc.py:614-655).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ldpc|qpsk_awgn|ofdm_siso|mimo_ofdm|pusch]
-                  [--cn-update boxplus-phi|minsum|...] [--impl reference]
+                  [--cn-update boxplus-phi|minsum|...] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Default workload `ldpc` = configs[1] (the configuration BASELINE.json's metric is quoted on): a "step" = one
@@ -32,6 +32,7 @@ EBNO_DB = 2.0
 # written once per iteration, one channel LLR read per VN per iteration, plus compulsory I/O.
 E_EDGES, N_VNS = 40320, 8832
 ALG_BYTES_PER_CW = NUM_ITER * (8 * E_EDGES + 4 * N_VNS) + 4 * N_CODE + 4 * K_INFO      # 7 208 448
+DUMP_BYTES = 60 << 20        # --dump-outputs: array data of all files together (< 64 MB with the .npy headers)
 
 
 def host_cores():
@@ -196,6 +197,9 @@ def run_reference(args):
         u_hat = dec(llr, num_threads=cores)
         errs += int(u_hat.sum())
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        import torch
+        dump_outputs(args.dump_outputs, {"u_hat": torch.from_numpy(np.asarray(u_hat))})
     val = sample * N_CODE * args.steps / dt
     line = {"metric": "coded bits/s, LDPC5G n=8448 k=4224 BP-20 decode", "value": val, "unit": "coded bits/s",
             "impl": "reference", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -221,6 +225,31 @@ def emit(line):
         sys.stdout.flush()
     else:
         os.write(_RESULT_FD, data)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes what the timed path returned in its last step as out_dir/<name>.npy, so that two builds of
+    the project can be compared output for output (the inputs are seeded: the same arguments give the same inputs).
+    float64 and int64 arrays are stored as float64, all others as float32, complex ones as trailing (real, imag) pairs.
+    An array larger than its share of DUMP_BYTES keeps a fixed, seeded sample of its rows, the same rows in every run."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    items = []
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.is_complex():
+            t = torch.view_as_real(t)
+        t = t.to(torch.float64 if t.dtype in (torch.float64, torch.int64) else torch.float32)
+        items.append((name, t.cpu().numpy()))
+    budget = DUMP_BYTES
+    for j, (name, a) in enumerate(sorted(items, key=lambda it: it[1].nbytes)):
+        share = budget // (len(items) - j)
+        if a.ndim and a.nbytes > share:
+            rows = np.random.default_rng(0).choice(a.shape[0], share // (a.nbytes // a.shape[0]), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        budget -= a.nbytes
 
 
 def time_calls(fn, reps, warm=2):
@@ -259,10 +288,10 @@ def dist_setup(args):
 # =====================================================================================================================
 # configs[0], [2], [3], [4]: receive chains (tools/bench_links.py)
 # =====================================================================================================================
-def measure_link(wl, steps, warmup, world, dev, e2e_steps=None, stage_reps=5):
+def measure_link(wl, steps, warmup, world, dev, e2e_steps=None, stage_reps=5, dump_dir=None):
     """Times `steps` passes of the workload's hot path (device time, max over ranks), its per-stage roofline table and
     the end-to-end leg with host buffers. Returns a dict of results (used by run_link and by the default line's
-    `config.other_workloads`)."""
+    `config.other_workloads`). With `dump_dir`, the last timed pass's output is written there (dump_outputs)."""
     import torch
     import torch.distributed as dist
     from sionna_b200 import _lib
@@ -279,12 +308,14 @@ def measure_link(wl, steps, warmup, world, dev, e2e_steps=None, stage_reps=5):
     l0 = _lib.lib().sb_launch_count()
     t0.record()
     for i in range(steps):
-        wl.run(i)
+        out = wl.run(i)
         if world > 1 and hasattr(wl, "counter"):
             dist.all_reduce(reduced.copy_(wl.counter.counters), op=dist.ReduceOp.SUM)
     t1.record()
     launches = _lib.lib().sb_launch_count() - l0
     torch.cuda.synchronize()
+    if dump_dir:
+        dump_outputs(dump_dir, {"output": out, **({"error_counters": wl.counter.counters} if hasattr(wl, "counter") else {})})
     if world > 1:
         dist.barrier()
     t = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device=dev)
@@ -355,7 +386,8 @@ def run_link(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    res = measure_link(wl, args.steps, max(args.warmup, 3), world, dev)
+    res = measure_link(wl, args.steps, max(args.warmup, 3), world, dev,
+                       dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if sampler else None
     link = None
     if hasattr(wl, "link_step"):                                  # PUSCH: the whole Monte-Carlo step incl. tx + channel
@@ -502,6 +534,8 @@ def run_ldpc(args):
         totals = reduced.cpu().tolist()
     else:
         totals = counter.counters.cpu().tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"u_hat": u_hat, "error_counters": counter.counters})
 
     # ---- end to end through the public API with HOST buffers: every step copies its logits from pinned host memory to
     # the device, decodes, and copies the decoded bits back to pinned host memory. Two streams are used round-robin so the
@@ -653,10 +687,14 @@ def main():
     ap.add_argument("--no-links", action="store_true", help="skip the short measurement of configs[0], [2], [3], [4]")
     ap.add_argument("--no-traffic", action="store_true", help="do not re-measure DRAM traffic with ncu")
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32 / float64, <= 64 MB in all)")
     ap.add_argument("--ebno-db", type=float, default=EBNO_DB,
                     help="Eb/N0 of the synthetic inputs (default 2 dB, SURVEY.md section 8d). The boxplus-phi kernel skips "
                          "provably-zero phi terms of saturated messages, so its speed depends on how early codewords converge")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.traffic_probe:
         return traffic_probe(args)
     sys.stdout.flush()

@@ -2,8 +2,9 @@
 
 Needs /root/reference (build container only). For every /root/reference/test/codes/ldpc/k{K}_n{N}_G.npy (the matrices
 the reference's own encoder test multiplies with, test/unit/fec/test_ldpc_encoding.py:97-148) draw 4 seeded random
-information words u, compute c = u G mod 2 with the golden G, and store (k, n, packbits(u), packbits(c)). The
-fixture (~150 KB) travels to the GPU box; the 18 MB of G matrices do not.
+information words u, compute c = u G mod 2 with the golden G, and store (k, n, packbits(u), packbits(c)). The smallest
+matrix (k = 64, n = 128) is also stored whole, as packbits(G), so that every row of the encoder can be checked. The
+fixture (~120 KB) is all the tests need; the 18 MB of G matrices are not part of the repository.
 """
 import os, re
 import numpy as np
@@ -26,6 +27,8 @@ for f in sorted(os.listdir(src)):
     c = (u.astype(np.int64) @ gm.astype(np.int64)) % 2
     out[f"u_{k}_{n}"] = np.packbits(u, axis=1)
     out[f"c_{k}_{n}"] = np.packbits(c.astype(np.uint8), axis=1)
+    if (k, n) == (64, 128):
+        out["g_64_128"] = np.packbits(gm, axis=1)
     params.append((k, n))
     print(k, n, gm.sum())
 out["params"] = np.array(params, np.int32)
